@@ -246,6 +246,23 @@ def config_dict(args, per_gpu_batch, where):
             **({"gradient_exchange": getattr(args, "dp_schedule", "")} if where != "cpu" and args.gpus > 1 else {})}
 
 
+DUMP_SAMPLE = 4 << 20          # parameter values written by --dump-outputs (float32: 16 MB)
+
+
+def dump_outputs(out_dir, ts, loss):
+    """What the last timed step handed back to its caller: the loss and the parameters the SGD update wrote, as
+    loss.npy (float64), param_norms.npy (float64 L2 norm of every parameter, in ts.parameters() order) and
+    param_sample.npy (float32, the same DUMP_SAMPLE positions of the concatenated parameters every run)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    params = [p.detach() for p in ts.parameters()]
+    np.save(os.path.join(out_dir, "loss.npy"), np.array([float(loss.detach())], dtype=np.float64))
+    np.save(os.path.join(out_dir, "param_norms.npy"), torch.stack([p.double().norm() for p in params]).cpu().numpy())
+    flat = torch.cat([p.reshape(-1).float() for p in params])
+    idx = torch.randint(0, flat.numel(), (min(DUMP_SAMPLE, flat.numel()),), generator=torch.Generator().manual_seed(0))
+    np.save(os.path.join(out_dir, "param_sample.npy"), flat[idx.sort().values.to(flat.device)].cpu().numpy())
+
+
 # --------------------------------------------------------------------------------------------------
 def run_ours(args, rank, world, local_rank):
     import adaptersis_b200 as asis
@@ -299,6 +316,8 @@ def run_ours(args, rank, world, local_rank):
     launches = _lib.launch_count() - n0 + args.steps * ts.graph_launches     # eager launches + kernel nodes replayed
     t_ms = e0.elapsed_time(e1)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, ts, loss)
 
     if args.only_timed:
         if rank == 0:
@@ -445,6 +464,8 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="launch every kernel eagerly instead of replaying the step's CUDA graph")
     ap.add_argument("--detail", action="store_true", help="print the per-shape GEMM breakdown of the profiled step")
     ap.add_argument("--only-timed", action="store_true", help="warm-up + timed loop only (used under ncu)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the loss and parameters of the last timed step as "
+                    "DIR/*.npy, to compare two builds on identical inputs")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 

@@ -1,4 +1,5 @@
-"""Seeded synthetic inputs shared by make_golden.py and the tests (no reference code involved)."""
+"""Seeded synthetic inputs and parameter initialisation shared by make_golden.py and the tests (no reference code
+involved)."""
 import torch
 
 ENCODER_DATA_SEED = 1900
@@ -20,6 +21,30 @@ def encoder_data(B=1, size=588, feat_channels=96, grid=42):
     target = (torch.rand(B, size, size, generator=gen) < 0.4).long()
     gfeat = torch.randn(B, feat_channels, grid, grid, generator=gen)
     return img, target, gfeat
+
+
+def stress_init(module, gen, scaled=False):
+    """Make every learnable path carry signal (default init leaves CAViT an identity, F4).
+    ``scaled``: the two MSDA projections get std 1.5/sqrt(fan_in) and 1/sqrt(fan_in) (offsets ~1.5 px, attention
+    logits ~1) instead of the fixed 0.3 / 0.5 of the dim-32 fixtures, which at larger widths would mean
+    +-several px offsets and one-hot softmaxes -- a chaotic map rather than a trained adapter."""
+    with torch.no_grad():
+        for name, p in module.named_parameters():
+            r = torch.randn(p.shape, generator=gen)
+            fan = p.shape[-1] ** 0.5 if p.dim() > 1 else 1.0
+            if name.endswith("gamma"):
+                p.copy_(0.5 + 0.2 * r)
+            elif "norm" in name and name.endswith("weight"):
+                p.copy_(1.0 + 0.1 * r)
+            elif "sampling_offsets.weight" in name:
+                p.copy_((1.5 / fan if scaled else 0.3) * r)
+            elif "attention_weights.weight" in name:
+                p.copy_((1.0 / fan if scaled else 0.5) * r)
+            elif name.endswith("bias") and "sampling_offsets" not in name:
+                p.copy_(0.05 * r)
+            elif name in ("cls_token", "mask_token"):
+                p.copy_(0.1 * r)
+    return module
 
 
 ADAPTER_DATA_SEED = 1700

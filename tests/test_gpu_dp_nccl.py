@@ -7,8 +7,8 @@ backbones/decoders.py uses nn.BatchNorm2d under DDP), which is a semantic differ
 gradient exchange; the decoder is therefore put in eval() for this comparison so that the only cross-sample
 couplings are the SyncBN layers, which DP must reproduce exactly.
 
-Needs >= 2 GPUs: skipped on the single-GPU test box; run with `gpurun --gpus 2 -- python -m pytest
-tests/test_gpu_dp_nccl.py` (result recorded in profiles/)."""
+Needs >= 2 GPUs and skips with fewer; on a machine with two, run `python -m pytest tests/test_gpu_dp_nccl.py`
+(result recorded in profiles/)."""
 import os
 import socket
 
@@ -87,7 +87,7 @@ def _worker(rank, world, port, precision, per_rank, overlap, q):
 @pytest.mark.parametrize("precision,tol,overlap", [("fp32", 1e-3, "0"), ("bf16", 2e-2, "0"), ("fp32", 1e-3, "1")])
 def test_two_gpu_gradients_equal_one_gpu(precision, tol, overlap):
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs 2 GPUs (gpurun --gpus 2)")
+        pytest.skip("needs 2 GPUs")
     world, per_rank = 2, 2
     ctx = mp.get_context("spawn")
     q = ctx.Queue()

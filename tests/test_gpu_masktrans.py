@@ -7,7 +7,7 @@ import pytest
 import torch
 import torch.nn.functional as F
 
-from conftest import relerr
+from conftest import grad_err, relerr
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda"
@@ -42,7 +42,7 @@ def test_mask_transformer_golden(golden, mode, tol, gtol):
     if mode == "fp32":
         assert torch.equal(pred, g["pred"])                                 # bit-exact
     assert torch.equal(pred[decided], g["pred"][decided])
-    bad = [(n, relerr(a.float(), g["grads"][n])) for n, a in zip(["input"] + names, grads) if not relerr(a.float(), g["grads"][n]) < gtol]
+    bad = [(n, grad_err(a, g["grads"][n])) for n, a in zip(["input"] + names, grads) if not grad_err(a, g["grads"][n]) < gtol]
     assert not bad, bad
 
 

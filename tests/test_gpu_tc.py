@@ -151,9 +151,9 @@ def test_composed_encoder_bf16_golden(golden):
     assert g["cfg"]["dim"] // g["cfg"]["heads"] == 64
     amp = g["amp_err"]
     r = run_composed(g, "bf16")
-    e_feat, e_x = relerr(r["feat"], g["feat"]), relerr(r["x"], g["x"])
+    e_feat, e_x = grad_err(r["feat"], g["feat"]), grad_err(r["x"], g["x"])
     logits = r["logits"].float()
-    e_log = relerr(logits[:, :, ::4, ::4], g["logits_s4"])
+    e_log = grad_err(logits[:, :, ::4, ::4], g["logits_s4"])
     print(f"[encoder_hd64.pt] bf16 mode: feat {e_feat:.2e} x {e_x:.2e} logits {e_log:.2e} "
           f"(reference under torch bf16 autocast: feat {amp['feat']:.2e} logits {amp['logits']:.2e})")
     assert e_feat < TOL and e_x < TOL
