@@ -19,7 +19,7 @@ NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 FLAGS = ["-O3", "-std=c++17", "-lineinfo", "--expt-relaxed-constexpr", "-Xcompiler", "-fPIC",
          "-Xptxas", "-v"]
-if os.environ.get("ASIS_TRACE"):      # debug build with in-kernel event stamps (tools/attn_trace.py, tools/gemm_trace.py):
+if os.environ.get("ASIS_TRACE"):      # debug build with in-kernel event stamps (tools/attn_trace8.py, tools/gemm_trace.py):
     FLAGS = FLAGS + ["-DASIS_TRACE"]  # a separate library, loaded with ASIS_LIB=<path>; the product library is untouched
     OUT = os.path.join(HERE, "libasis_b200_trace.so")
     BUILD = os.path.join(CSRC, "build_trace")

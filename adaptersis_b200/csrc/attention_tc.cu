@@ -4,7 +4,7 @@
 // dropout); T = 1765 is not a multiple of the 128-row tiles: TMA zero-fills rows >= T and the
 // softmax masks key columns >= T.
 //
-// Forward (attn_fwd8_kernel; the earlier v7b is kept as attn_fwd_kernel behind ASIS_ATTN_FWD=7): persistent CTAs walk
+// Forward (attn_fwd8_kernel): persistent CTAs walk
 //   items = PAIRS of 128-query tiles of one (image, head).  Warps 0-3 / 4-7 are two softmax warpgroups (1 thread = 1 TMEM
 //   lane = 1 query row), warpgroup w owns query tile 2*pair + w over all key tiles; warp 8 = TMA producer (K and V rings,
 //   double-buffered Q pair), warp 9 = MMA issuer, event driven (polls the barriers of both warpgroups).  TMEM per
@@ -27,7 +27,6 @@ constexpr int BWD_THREADS = 576;      // backward: TMA warp, MMA warp, 2 x 8 sof
 constexpr int TILE = 128;      // query / key rows per tile
 constexpr int HD = 64;
 constexpr int T16K = TILE * HD * 2;           // one 128 x 64 bf16 tile
-constexpr int T32K = TILE * TILE * 2;         // one 128 x 128 bf16 tile (two 128 x 64 sub-tiles)
 constexpr float LOG2E = 1.4426950408889634f;
 constexpr float LN2 = 0.6931471805599453f;
 
@@ -35,13 +34,6 @@ __device__ __forceinline__ float fast_exp2(float x) {
   float y;
   asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
   return y;
-}
-
-__device__ __forceinline__ void named_bar_sync(int id, int nthreads) {
-  asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
-}
-__device__ __forceinline__ void named_bar_arrive(int id, int nthreads) {
-  asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
 }
 
 // write 32 consecutive bf16 of row `row` (columns [col0, col0+32), col0 % 32 == 0) into a K-major,
@@ -154,11 +146,9 @@ struct AttnParams {
 constexpr int HALF = 64;                     // key / query tile width of the backward kernels
 constexpr int T8K = HALF * HD * 2;           // one 64 x 64 bf16 tile
 constexpr uint32_t TMEM_COLS = 512;
+constexpr int NSB = 3;              // backward: rotating score buffers in TMEM (tile j uses buffer j % 3)
 
-// ------------------------------------------------------------------------------------------------
-// forward
-// ------------------------------------------------------------------------------------------------
-// ---- optional event trace (built with -DASIS_TRACE only: tools/attn_trace.py) ---------------------
+// ---- optional event trace (built with -DASIS_TRACE only: tools/attn_trace8.py, tools/attn_bwd_trace.py) -------------
 #ifdef ASIS_TRACE
 __device__ unsigned long long *g_attn_trace = nullptr;     // [16 slots][1024] clock64 stamps of CTA 0
 #define ATTN_TRACE(slot, idx)                                                                  \
@@ -169,348 +159,10 @@ __device__ unsigned long long *g_attn_trace = nullptr;     // [16 slots][1024] c
 #define ATTN_TRACE(slot, idx) do { } while (0)
 #endif
 
-constexpr int FWD_STAGES = 4;
-constexpr int NSB = 3;              // rotating score buffers in TMEM (global tile g uses buffer g % 3)
-constexpr int FWD_SMEM = 2 * T16K /*Q, double buffered*/ + FWD_STAGES * 2 * T16K /*K,V*/ + T32K /*merge exchange*/ +
-                         1024 /*(m, l) exchange*/ + 1024 /*align*/ + 512 /*barriers*/;
-
-// Persistent: one CTA per SM walks over its (query block, head, image) items; the TMA and MMA warps
-// run ahead across item boundaries (next Q into the other Q buffer, next K/V into the ring, the first
-// score tiles of the next item into the free TMEM buffers) while the softmax warpgroups finish the
-// current item -- with one CTA per item the softmax warps spent ~20 % of their time waiting for the
-// first scores and the tensor pipe idled through every prologue / epilogue.
-__global__ void __launch_bounds__(ATT_THREADS, 1)
-attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQKV, const AttnParams p, const int num_items, const int nqb) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t *smem = reinterpret_cast<uint8_t *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-  uint8_t *sQ = smem;                            // 2 tiles
-  uint8_t *sK = sQ + 2 * T16K;                   // FWD_STAGES tiles
-  uint8_t *sV = sK + FWD_STAGES * T16K;          // FWD_STAGES tiles
-  uint8_t *sX = sV + FWD_STAGES * T16K;          // merge exchange: [64][128] fp32 partial O of warpgroup 1
-  float *sML = reinterpret_cast<float *>(sX + T32K);       // [2][128]: warpgroup 1's (m, l)
-  uint64_t *bars = reinterpret_cast<uint64_t *>(sX + T32K + 1024);
-  uint64_t *q_full = bars, *q_empty = q_full + 2, *k_full = q_empty + 2, *k_empty = k_full + FWD_STAGES,
-           *v_full = k_empty + FWD_STAGES, *v_empty = v_full + FWD_STAGES, *s_full = v_empty + FWD_STAGES,
-           *p_full = s_full + NSB, *o_full = p_full + 2, *o_empty = o_full + 2, *x_free = o_empty + 2;
-  uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(x_free + 1);
-
-  // Roles by warp id: 0-3 softmax warpgroup 0, 4-7 softmax warpgroup 1, 8 TMA producer, 9 MMA issuer.
-  // The SMSP arbiter favours the highest warp id: with the MMA warp as warp 1 it shared its scheduler
-  // with two busy softmax warps of higher priority and every P V / S issue waited for their stalls.
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  constexpr int TMA_WARP = 8, MMA_WARP = 9;
-#ifdef ASIS_TRACE
-  unsigned long long *tr = g_attn_trace;
-#endif
-  const int C = p.H * HD;
-  const int nkv = (p.T + TILE - 1) / TILE;
-  const int n_my = (num_items - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;   // items of this CTA
-  const int G = n_my * nkv;                                                               // its key tiles, in order
-
-  if (warp == TMA_WARP && lane == 0) {
-    tma_prefetch_desc(&tmQKV);
-    for (int i = 0; i < 2; ++i) {
-      mbar_init(q_full + i, 1);
-      mbar_init(q_empty + i, 1);
-      mbar_init(p_full + i, 4);
-      mbar_init(o_full + i, 1);
-      mbar_init(o_empty + i, 4);
-    }
-    for (int i = 0; i < FWD_STAGES; ++i) {
-      mbar_init(k_full + i, 1);
-      mbar_init(k_empty + i, 1);
-      mbar_init(v_full + i, 1);
-      mbar_init(v_empty + i, 1);
-    }
-    for (int i = 0; i < NSB; ++i) mbar_init(s_full + i, 1);
-    mbar_init(x_free, 4);
-    fence_barrier_init();
-  }
-  if (warp == MMA_WARP) tmem_alloc(tmem_slot, TMEM_COLS);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem = *tmem_slot;
-  // S[b] at b*128 (b < 3); the bf16 probabilities P overwrite columns [0, 64) of their own score
-  // buffer (two keys per 32-bit column) and feed the second GEMM as its A operand straight from TMEM;
-  // O[w] at 384 + w*64.  Keeping P out of shared memory matters: with P staged in smem every key tile
-  // moved 144 KB through the 128 B/clk shared-memory port (Q+K and P+V operand reads, the P stores,
-  // the TMA fills) = 1150 clk against 512 clk of MMA -- the kernel was shared-memory bound.
-  const uint32_t tS = tmem, tO = tmem + NSB * TILE;
-
-  // The TMA and MMA roles run warp-uniformly (every lane executes the loops and the barrier waits;
-  // only the TMA / tcgen05 instructions sit under elect_one): operands then live in uniform registers
-  // and the MMAs issue back to back instead of through per-instruction R2UR waterfall loops.
-  if (warp == TMA_WARP) {
-    // K and V travel in separate rings: a K stage is free as soon as its score MMA has run (three
-    // tiles before the P V that frees the V stage), and the K loads are issued KLEAD tiles ahead of
-    // the V loads.  With one shared ring the K tile of S(g+3) could only be requested when P V(g-1)
-    // had finished, and the MMA warp (hence every later P V) sat waiting for it.
-    constexpr int KLEAD = 3;
-    for (int i = 0; i < G + KLEAD; ++i) {
-      if (i < G) {
-        const int k = i / nkv, j = i - k * nkv;
-        const int item = (int)blockIdx.x + k * (int)gridDim.x;
-        const int bh = item / nqb, qb = item - bh * nqb, h = bh % p.H, b = bh / p.H;
-        if (j == 0) {
-          const int qbuf = k & 1;
-          if (k >= 2) mbar_wait(q_empty + qbuf, ((k >> 1) - 1) & 1);
-          if (elect_one()) {
-            mbar_arrive_expect_tx(q_full + qbuf, T16K);
-            tma_load_3d(&tmQKV, q_full + qbuf, sQ + qbuf * T16K, h * HD, qb * TILE, b);
-          }
-          __syncwarp();
-        }
-        const int st = i % FWD_STAGES, use = i / FWD_STAGES;
-        if (use > 0) mbar_wait(k_empty + st, (use - 1) & 1);
-        if (elect_one()) {
-          mbar_arrive_expect_tx(k_full + st, T16K);
-          tma_load_3d(&tmQKV, k_full + st, sK + st * T16K, C + h * HD, j * TILE, b);
-        }
-        __syncwarp();
-      }
-      const int g = i - KLEAD;
-      if (g >= 0) {
-        const int k = g / nkv, j = g - k * nkv;
-        const int item = (int)blockIdx.x + k * (int)gridDim.x;
-        const int bh = item / nqb, h = bh % p.H, b = bh / p.H;
-        const int st = g % FWD_STAGES, use = g / FWD_STAGES;
-        if (use > 0) mbar_wait(v_empty + st, (use - 1) & 1);
-        if (elect_one()) {
-          mbar_arrive_expect_tx(v_full + st, T16K);
-          tma_load_3d(&tmQKV, v_full + st, sV + st * T16K, 2 * C + h * HD, j * TILE, b);
-        }
-        __syncwarp();
-      }
-    }
-  } else if (warp == MMA_WARP) {
-    constexpr uint32_t idesc_s = make_idesc(TILE, TILE, 0, 0);   // S = Q K^T : both K-major
-    constexpr uint32_t idesc_o = make_idesc(TILE, HD, 0, 1);     // O = P V   : V is MN-major
-    // This warp's loop is the pacemaker of the whole CTA (a timeline of the first persistent version
-    // showed ~1500 clk per key tile spent here: two integer divisions, 12 descriptors rebuilt with
-    // shifts and masks in the uniform datapath, ...), so everything is carried incrementally: the
-    // descriptors are base + constant (the 14-bit address field cannot carry: smem < 256 KB), the
-    // (item, tile, buffer, stage, phase) counters of the score stream and of the P V stream are
-    // stepped, never divided.
-    const uint64_t dQ = desc_kmajor(smem_u32(sQ), 0), dK = desc_kmajor(smem_u32(sK), 0), dV = desc_mnmajor(smem_u32(sV), 0);
-    constexpr uint32_t STAGE16 = T16K >> 4;                      // one 16 KB tile in descriptor address units
-    // Scores go round three TMEM buffers and are issued three tiles ahead of the P V that consumes
-    // them, across item boundaries.  S(g) overwrites the buffer P V(g-3) read its A operand from:
-    // both are issued by this warp in that order and tcgen05.mma executes in issue order.
-    struct Stream { int g, k, j, sb, st; uint32_t ph; } ss{0, 0, 0, 0, 0, 0}, ps{0, 0, 0, 0, 0, 0};   // ph: phase of the K / V stage ring
-    auto step = [&](Stream &x) {
-      ++x.g;
-      if (++x.j == nkv) { x.j = 0; ++x.k; }
-      if (++x.sb == NSB) x.sb = 0;
-      if (++x.st == FWD_STAGES) { x.st = 0; x.ph ^= 1; }
-    };
-    auto issue_s = [&]() {
-      const int qbuf = ss.k & 1;
-      if (ss.j == 0) mbar_wait(q_full + qbuf, (ss.k >> 1) & 1);
-      mbar_wait(k_full + ss.st, ss.ph);
-      tc_fence_after();
-      if (elect_one()) {
-        const uint64_t a = dQ + (uint32_t)(qbuf * STAGE16), bdesc = dK + (uint32_t)(ss.st * STAGE16);
-        const uint32_t d = tS + ss.sb * TILE;
-#pragma unroll
-        for (int kk = 0; kk < 4; ++kk) umma_bf16(d, a + 2 * kk, bdesc + 2 * kk, idesc_s, kk > 0);
-        umma_commit(s_full + ss.sb);
-        umma_commit(k_empty + ss.st);
-        if (ss.j == nkv - 1) umma_commit(q_empty + qbuf);      // the Q buffer may be refilled (item k + 2)
-      }
-      __syncwarp();
-      ATTN_TRACE(2, ss.g);
-      step(ss);
-    };
-    for (int i = 0; i < NSB && i < G; ++i) issue_s();
-    for (; ps.g < G; step(ps)) {
-      const int w = ps.g & 1;
-      mbar_wait(v_full + ps.st, ps.ph);
-      mbar_wait(p_full + w, (ps.g >> 1) & 1);
-      ATTN_TRACE(0, ps.g);
-      if (ps.j == 0 && ps.k > 0) {                             // both warpgroups have read the previous item's O
-        mbar_wait(o_empty + 0, (ps.k - 1) & 1);
-        mbar_wait(o_empty + 1, (ps.k - 1) & 1);
-      }
-      tc_fence_after();
-      if (elect_one()) {
-        const uint64_t bdesc = dV + (uint32_t)(ps.st * STAGE16);
-        const uint32_t d = tO + w * HD, a = tS + ps.sb * TILE;
-        const uint32_t acc0 = ps.j >= 2;
-#pragma unroll
-        for (int kk = 0; kk < 8; ++kk)     // O[w] (+)= P V, accumulated in TMEM over this warpgroup's tiles of the item
-          umma_bf16_ts(d, a + kk * 8, bdesc + 128 * kk, idesc_o, kk > 0 ? 1u : acc0);
-        umma_commit(o_full + w);
-        umma_commit(v_empty + ps.st);
-      }
-      __syncwarp();
-      ATTN_TRACE(1, ps.g);
-      if (ss.g < G) issue_s();
-    }
-  } else {
-    const int w = warp >> 2;                        // warpgroup: global key tiles g == w (mod 2)
-    const int quarter = warp & 3;
-    const int row = quarter * 32 + lane;            // row inside the tile == TMEM lane
-    const uint32_t lane_addr = (uint32_t)(quarter * 32) << 16;
-    // (A named-barrier ping-pong that made the two warpgroups' exponential phases mutually exclusive
-    // was measured and is slower: a warp issues in order and ptxas bunches the MUFU.EX2s, so a lone
-    // warp serialises its MUFU and FMA work -- 2050 clk per tile -- whereas two warps of different
-    // warpgroups on one scheduler fill each other's gaps -- 2200 clk for two tiles.)
-    for (int k = 0; k < n_my; ++k) {
-      float *xch = reinterpret_cast<float *>(sX);     // [64][128] floats
-      float *ml = sML;
-      const int item = (int)blockIdx.x + k * (int)gridDim.x;
-      const int qb = item % nqb, bh = item / nqb, h = bh % p.H, b = bh / p.H;
-      const int g0 = k * nkv;
-      // Running state in the log2 domain.  O[w] lives in TMEM and is accumulated there by the MMAs; it
-      // is only touched here when the running maximum grows by more than 2^8 (lazy rescaling: until
-      // then the probabilities are formed against the stale maximum m_use, at most 256x too large --
-      // harmless in fp32 / bf16 -- and (m_use, l, O) stay mutually consistent).
-      float m_use = -INFINITY, l_run = 0.f;
-      int u = 0, g_last = -1;
-      for (int g = g0 + ((g0 ^ w) & 1); g < g0 + nkv; g += 2, ++u) {
-        const int kv0 = (g - g0) * TILE;
-        const int sb = g % NSB;
-        g_last = g;
-        if (quarter == 0) ATTN_TRACE(4, g);
-        mbar_wait(s_full + sb, (g / NSB) & 1);
-        tc_fence_after();
-        if (quarter == 0) ATTN_TRACE(5, g);
-        // the whole score row into registers with one wait; the TMEM buffer is free again right away
-        float s[4][32];
-#pragma unroll
-        for (int c = 0; c < 4; ++c) tmem_ld32_issue(tS + lane_addr + sb * TILE + c * 32, s[c]);
-        tmem_ld_wait();
-        if (quarter == 0) ATTN_TRACE(6, g);
-        if (kv0 + TILE > p.T) {                          // only the last key block has invalid columns
-#pragma unroll
-          for (int c = 0; c < 4; ++c)
-#pragma unroll
-            for (int i = 0; i < 32; ++i)
-              if (kv0 + c * 32 + i >= p.T) s[c][i] = -INFINITY;
-        }
-        float mx4[4];
-#pragma unroll
-        for (int c = 0; c < 4; ++c) {
-          mx4[c] = fmaxf(s[c][0], s[c][1]);
-#pragma unroll
-          for (int i = 2; i < 32; i += 2) mx4[c] = fmaxf(mx4[c], fmaxf(s[c][i], s[c][i + 1]));
-        }
-        const float m_new = fmaxf(m_use, fmaxf(fmaxf(mx4[0], mx4[1]), fmaxf(mx4[2], mx4[3])) * p.scale_log2);
-        if (quarter == 0) ATTN_TRACE(7, g);
-        if (u == 0) {
-          m_use = m_new;
-        } else {
-          const bool grow = m_new - m_use > 8.f;
-          if (__any_sync(0xffffffffu, grow)) {
-            const float alpha = grow ? fast_exp2(m_use - m_new) : 1.f;
-            if (grow) m_use = m_new;
-            l_run *= alpha;
-            mbar_wait(o_full + w, ((g >> 1) - 1) & 1);     // every P V issued so far for this warpgroup is complete
-            tc_fence_after();
-#pragma unroll 1
-            for (int c = 0; c < 2; ++c) {                // 32 columns at a time: the score row owns the registers
-              float o0[32];
-              tmem_ld32(tO + lane_addr + w * HD + c * 32, o0);
-#pragma unroll
-              for (int i = 0; i < 32; ++i) o0[i] *= alpha;
-              tmem_st32(tO + lane_addr + w * HD + c * 32, o0);
-            }
-            tmem_st_wait();
-          }
-        }
-        if (quarter == 0) ATTN_TRACE(8, g);
-        // Observe EVERY phase of o_full[w] in order (this warpgroup's previous P V has completed), even
-        // though P no longer lives in a buffer that P V reads.  The waits are by phase parity: a warp that
-        // skipped them could reach the item epilogue with the barrier still one phase behind (P V(g-2) not
-        // complete -- s_full(g) only implies P V(g-3)), where the parity of "P V(g_last) done" equals the
-        // parity of the phase before P V(g-2): the wait passes at once and O[w] is read before the last
-        // two key tiles have been accumulated (32-row blocks off by ~1e-2, run-to-run different -- found
-        // with tools/attn_stress.py).  It is normally already satisfied: P V(g-2) was issued a tile ago.
-        if (u > 0) {
-          mbar_wait(o_full + w, ((g >> 1) - 1) & 1);
-          tc_fence_after();
-        }
-        float l4[4] = {0.f, 0.f, 0.f, 0.f};
-#pragma unroll
-        for (int half = 0; half < 2; ++half) {
-          uint32_t pk[32];                               // keys [64 half, 64 half + 64), two per word
-#pragma unroll
-          for (int c = 0; c < 2; ++c)
-#pragma unroll
-            for (int i = 0; i < 32; i += 2) {
-              const float e0 = fast_exp2(fmaf(s[2 * half + c][i], p.scale_log2, -m_use));
-              const float e1 = fast_exp2(fmaf(s[2 * half + c][i + 1], p.scale_log2, -m_use));
-              l4[(i >> 1) & 3] += e0 + e1;
-              __nv_bfloat162 hh = __floats2bfloat162_rn(e0, e1);
-              pk[c * 16 + (i >> 1)] = *reinterpret_cast<uint32_t *>(&hh);
-            }
-          tmem_st32u(tS + lane_addr + sb * TILE + half * 32, pk);
-        }
-        l_run += (l4[0] + l4[1]) + (l4[2] + l4[3]);
-        if (quarter == 0) ATTN_TRACE(9, g);
-        tmem_st_wait();
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(p_full + w);
-        if (quarter == 0) ATTN_TRACE(10, g);
-      }
-      // ---- item epilogue: read O[w], release it, merge the two warpgroups' partial softmax states
-      float o[64];
-      if (u > 0) {
-        mbar_wait(o_full + w, (g_last >> 1) & 1);
-        tc_fence_after();
-#pragma unroll
-        for (int c = 0; c < 2; ++c) {
-          float v[32];
-          tmem_ld32(tO + lane_addr + w * HD + c * 32, v);
-#pragma unroll
-          for (int i = 0; i < 32; ++i) o[c * 32 + i] = v[i];
-        }
-      } else {
-#pragma unroll
-        for (int i = 0; i < 64; ++i) o[i] = 0.f;
-      }
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(o_empty + w);           // the next item's first P V may overwrite O[w]
-      if (w == 1) {
-        if (k > 0) mbar_wait(x_free, (k - 1) & 1);       // warpgroup 0 has consumed the previous item's exchange
-        ml[row] = m_use;
-        ml[128 + row] = l_run;
-#pragma unroll
-        for (int i = 0; i < 64; ++i) xch[i * 128 + row] = o[i];
-      }
-      named_bar_sync(1, 256);
-      if (w == 0) {
-        const float m1 = ml[row], l1 = ml[128 + row];
-        const float m = fmaxf(m_use, m1);
-        const float a0 = (m_use == -INFINITY) ? 0.f : fast_exp2(m_use - m), a1 = (m1 == -INFINITY) ? 0.f : fast_exp2(m1 - m);
-        const float l = l_run * a0 + l1 * a1;
-#pragma unroll
-        for (int i = 0; i < 64; ++i) o[i] = o[i] * a0 + xch[i * 128 + row] * a1;
-        __syncwarp();
-        if (lane == 0) mbar_arrive(x_free);
-        const int t = qb * TILE + row;
-        if (t < p.T) {
-          store_out64(p.out + ((size_t)b * p.T + t) * C + h * HD, o, 1.f / l);
-          p.lse[((size_t)b * p.H + h) * p.T + t] = (m + log2f(l)) * LN2;
-        }
-      }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == MMA_WARP) {
-    tc_fence_after();
-    tmem_dealloc(tmem, TMEM_COLS);
-  }
-}
-
 // ------------------------------------------------------------------------------------------------
 // forward, version 8: every softmax warpgroup OWNS a query tile
 // ------------------------------------------------------------------------------------------------
-// A timeline of v7b (tools/attn_trace.py; profiles/r2_attn_trace.md) showed two things.  (1) The exponential phase of a
+// A timeline of the previous forward (v7b) showed two things.  (1) The exponential phase of a
 // key tile takes a warp ~2050 clk = exactly the MUFU throughput when the other warpgroup's warp on the same scheduler
 // is in its own exponential phase (2 x 128 MUFU.EX2 x 8 clk): the kernel is MUFU bound while it runs.  (2) It does not
 // run all the time: the two warpgroups split the KEY tiles of one query tile, so at the end of every item (14 key
@@ -525,7 +177,7 @@ constexpr int F8_STAGES = 4;
 constexpr int F8_SMEM = 2 * 2 * T16K /*Q: 2 warpgroups x 2 buffers*/ + F8_STAGES * 2 * T16K /*K, V rings*/ + 1024 /*align*/ + 512 /*barriers*/;
 
 __global__ void __launch_bounds__(ATT_THREADS, 1)
-attn_fwd8_kernel(const __grid_constant__ CUtensorMap tmQKV, const AttnParams p, const int num_items, const int npair, const int stagger) {
+attn_fwd8_kernel(const __grid_constant__ CUtensorMap tmQKV, const AttnParams p, const int num_items, const int npair) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t *smem = reinterpret_cast<uint8_t *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
   uint8_t *sQ = smem;                            // [buffer][warpgroup] tiles
@@ -541,7 +193,7 @@ attn_fwd8_kernel(const __grid_constant__ CUtensorMap tmQKV, const AttnParams p, 
 #ifdef ASIS_TRACE
   unsigned long long *tr = g_attn_trace;
 #endif
-  constexpr int TMA_WARP = 8, MMA_WARP = 9;      // the SMSP arbiter favours the highest warp id (see v7b)
+  constexpr int TMA_WARP = 8, MMA_WARP = 9;      // the SMSP arbiter favours the highest warp id
   const int C = p.H * HD;
   const int nkv = (p.T + TILE - 1) / TILE;
   const int n_my = (num_items - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;
@@ -702,20 +354,12 @@ attn_fwd8_kernel(const __grid_constant__ CUtensorMap tmQKV, const AttnParams p, 
     const int row = quarter * 32 + lane;            // row inside the tile == TMEM lane
     const uint32_t lane_addr = (uint32_t)(quarter * 32) << 16;
     const uint32_t tS = tmem + lane_addr + w * WG_COLS, tP = tS + P_OFF, tO = tS + O_OFF;
-    // Optional initial phase shift between the warpgroups (experiment knob, ASIS_ATTN_STAGGER, default off).  Every
-    // scheduler hosts one warp of each warpgroup; the idea was that, half a period apart, one warp's MUFU-bound
-    // exponential phase covers the other's issue-bound load / max / wait phases.  Measured: no effect at any shift --
-    // a warp's exponential phase takes ~2000 clk whether or not the other warp of its scheduler is in the same phase.
-    if (w == 1 && stagger > 0) {
-      const long long t0 = clock64();
-      while (clock64() - t0 < stagger) { }
-    }
     for (int k = 0; k < n_my; ++k) {
       const int item = (int)blockIdx.x + k * (int)gridDim.x;
       const int pr = item % npair, bh = item / npair, h = bh % p.H, b = bh / p.H;
       const int g0 = k * nkv;
       // running state in the log2 domain; O_w lives in TMEM and is only touched here when the running maximum grows
-      // by more than 2^8 (lazy rescaling, as in v7b)
+      // by more than 2^8 (lazy rescaling)
       float m_use = -INFINITY, l_run = 0.f;
       for (int j = 0; j < nkv; ++j) {
         const int g = g0 + j;
@@ -785,7 +429,7 @@ attn_fwd8_kernel(const __grid_constant__ CUtensorMap tmQKV, const AttnParams p, 
         if (quarter == 0) ATTN_TRACE(7 + 6 * w, g);       // exponentials done
         if (j > 0) {
           // P V(g-1) complete: O_w is consistent and the P columns are free.  Every phase of o_full[w] is observed
-          // in order (here, or at the end of the item), so the parity waits cannot alias (see v7b's post-mortem).
+          // in order (here, or at the end of the item), so the parity waits cannot alias.
           mbar_wait_wd(o_full + w, (g - 1) & 1);
           tc_fence_after();
           if (__any_sync(0xffffffffu, grow)) {
@@ -1277,7 +921,6 @@ int attention_tc_forward(const void *qkv, void *out, float *lse, int B, int T, i
   if (int rc = make_tmap_3d(&tq, qkv, 3 * C, T, B, 3 * C, (uint64_t)T * 3 * C, HD, TILE, 1)) return rc;
   static bool configured = false;
   if (!configured) {
-    if (int rc = set_smem((const void *)attn_fwd_kernel, FWD_SMEM)) return rc;
     if (int rc = set_smem((const void *)attn_fwd8_kernel, F8_SMEM)) return rc;
     configured = true;
   }
@@ -1288,27 +931,10 @@ int attention_tc_forward(const void *qkv, void *out, float *lse, int B, int T, i
   p.out = (bf16 *)out;
   p.lse = lse;
   const int nqb = (T + TILE - 1) / TILE;
-  static int version = -1;      // ASIS_ATTN_FWD=7: the v7b kernel (warpgroups split the key tiles), kept for comparison
-  if (version < 0) {
-    const char *e = getenv("ASIS_ATTN_FWD");
-    version = e ? atoi(e) : 8;
-  }
-  if (version == 7) {
-    const int num_items = nqb * H * B;
-    const int grid = num_items < sm_count() ? num_items : sm_count();
-    attn_fwd_kernel<<<grid, ATT_THREADS, FWD_SMEM, st>>>(tq, p, num_items, nqb);
-    ASIS_LAUNCHED();
-    return ASIS_OK;
-  }
   const int npair = (nqb + 1) / 2;
   const int num_items = npair * H * B;
   const int grid = num_items < sm_count() ? num_items : sm_count();
-  static int stagger = -1;      // ASIS_ATTN_STAGGER: initial delay of warpgroup 1 in clocks (see the kernel)
-  if (stagger < 0) {
-    const char *e = getenv("ASIS_ATTN_STAGGER");
-    stagger = e ? atoi(e) : 0;        // measured 0 / 800 / 1600 / 2400 clk: 275.6 / 276.7 / 280.0 / 277.1 us -- no effect, off
-  }
-  attn_fwd8_kernel<<<grid, ATT_THREADS, F8_SMEM, st>>>(tq, p, num_items, npair, stagger);
+  attn_fwd8_kernel<<<grid, ATT_THREADS, F8_SMEM, st>>>(tq, p, num_items, npair);
   ASIS_LAUNCHED();
   return ASIS_OK;
 }

@@ -9,12 +9,11 @@
 //   warp 9      MMA issuer     tcgen05.mma.kind::f16, fp32 accumulators in TMEM (2 x 256 columns, double buffered)
 // Three mbarrier pipelines: smem full/empty (TMA <-> MMA), TMEM full/empty (MMA <-> epilogue).
 //
-// gemm_tc_pair_kernel (the one the step runs): the two CTAs of a cluster form ONE 256 x 256 tcgen05.mma.cta_group::2
+// gemm_tc_pair_kernel (every GEMM with M > 128): the two CTAs of a cluster form ONE 256 x 256 tcgen05.mma.cta_group::2
 //   tile (6 x 32 KB ring per CTA: its 128 rows of A + half of the B tile); one instantiation per hot
 //   (A-major, B-major, epilogue kind, output dtype, saved-branch flag) combination plus an all-in-one fallback;
 //   also runs the implicit 3x3 convolutions (gemm_tc_conv3x3: taps as TMA row shifts over zero-padded maps).
-// gemm_tc_kernel<.., CL> (M < 256, comparison): 128 x 256 cta_group::1 tiles, clusters of CL CTAs along M share the B tile
-//   by TMA multicast (4 x 48 KB ring).
+// gemm_tc_kernel<A_MN, B_MN> (M <= 128: one M tile): 128 x 256 cta_group::1 tiles, one CTA each (4 x 48 KB ring).
 // Tails in M, N and K come for free from TMA zero fill; stores are masked.
 //
 // Both operands may be K-major (nn.Linear forward: x[R,K], W[N,K]) or MN-major (input gradient:
@@ -477,7 +476,10 @@ __device__ __forceinline__ void epi_slab3(const GemmTcParams &p, uint32_t taddr,
   }
 }
 
-template <int A_MN, int B_MN, int CL>
+// ---- 1-CTA kernel (tcgen05.mma.cta_group::1), GEMMs with M <= 128 -------------------------------------------
+// One 128 x 256 tile per CTA (4 x 48 KB ring).  With a single M tile the pair kernel would spend its second CTA on zero
+// rows: on the step's M <= 128 weight gradients it measured 0-8 % slower than this kernel (DESIGN.md section 5.2).
+template <int A_MN, int B_MN>
 __global__ void __launch_bounds__(GEMM_THREADS, 1)
 gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const GemmTcParams p) {
   extern __shared__ uint8_t smem_raw[];
@@ -489,20 +491,15 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   uint64_t *tempty_bar = tfull_bar + 2;
   uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(tempty_bar + 2);
 
-  // Roles by warp id: 0-7 epilogue, 8 TMA producer, 9 MMA issuer.  The SMSP arbiter favours the
-  // highest warp id, so the latency-critical single-warp roles get the top ids.
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   constexpr int TMA_WARP = NUM_EPI_WARPS, MMA_WARP = NUM_EPI_WARPS + 1;
-  const int crank = CL > 1 ? (int)cluster_ctarank() : 0;
-  const int cluster_id = blockIdx.x / CL, num_clusters = gridDim.x / CL;
-  constexpr uint16_t kMask = (uint16_t)((1u << CL) - 1u);
 
   if (warp == TMA_WARP && lane == 0) {
     tma_prefetch_desc(&tmA);
     tma_prefetch_desc(&tmB);
     for (int s = 0; s < STAGES; ++s) {
       mbar_init(full_bar + s, 1);
-      mbar_init(empty_bar + s, CL);   // every CTA of the cluster releases the stage (they all write into it)
+      mbar_init(empty_bar + s, 1);
     }
     for (int a = 0; a < 2; ++a) {
       mbar_init(tfull_bar + a, 1);
@@ -513,22 +510,17 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   if (warp == MMA_WARP) tmem_alloc(tmem_slot, 512);
   tc_fence_before();
   __syncthreads();
-  if (CL > 1) cluster_sync_all();     // peers' barriers are initialised before anything remote touches them
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
 
-  const int total_tiles = p.m_groups * p.n_tiles * p.splits;   // per cluster: CL adjacent m-tiles at once
+  const int total_tiles = p.m_groups * p.n_tiles * p.splits;
 
-  // Producer and MMA roles run WARP-UNIFORMLY (all 32 lanes execute the loops and the barrier waits;
-  // only the TMA / tcgen05 instructions themselves sit under elect_one).  With the whole role under
-  // `if (lane == 0)` the loop state lives in per-thread registers and every TMA / MMA operand has
-  // to be moved to uniform registers through an ELECT / R2UR.BROADCAST waterfall loop: the MMA
-  // thread then needs ~100 issue cycles per 128-cycle MMA and the tensor pipe starves.
+  // (warp-uniform producer and MMA roles: see the pair kernel)
   if (warp == TMA_WARP) {
     int stage = 0;
     uint32_t phase = 0;
-    for (int tile = cluster_id; tile < total_tiles; tile += num_clusters) {
-      const int m_blk = (tile % p.m_groups) * CL + crank;
+    for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x) {
+      const int m_blk = tile % p.m_groups;
       const int rest = tile / p.m_groups;
       const int n_blk = rest % p.n_tiles;
       const int split = rest / p.n_tiles;
@@ -539,7 +531,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         if (lane == 0) {
           uint8_t *sa = smem + stage * STAGE_BYTES;
           uint8_t *sb = sa + A_BYTES;
-          mbar_arrive_expect_tx(full_bar + stage, STAGE_BYTES);   // own A + the CL slices of B
+          mbar_arrive_expect_tx(full_bar + stage, STAGE_BYTES);
           if (A_MN == 0) {
             tma_load_2d(&tmA, full_bar + stage, sa, kb * BK, m_blk * BM);
           } else {
@@ -547,25 +539,12 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             for (int j = 0; j < BM / 64; ++j)
               tma_load_2d(&tmA, full_bar + stage, sa + j * BOX_BYTES, m_blk * BM + j * 64, kb * BK);
           }
-          if (CL == 1) {
-            if (B_MN == 0) {
-              tma_load_2d(&tmB, full_bar + stage, sb, kb * BK, n_blk * BN);
-            } else {
-#pragma unroll
-              for (int j = 0; j < BN / 64; ++j)
-                tma_load_2d(&tmB, full_bar + stage, sb + j * BOX_BYTES, n_blk * BN + j * 64, kb * BK);
-            }
+          if (B_MN == 0) {
+            tma_load_2d(&tmB, full_bar + stage, sb, kb * BK, n_blk * BN);
           } else {
-            // this CTA's 1/CL slice of B, multicast to the whole cluster
-            constexpr int ROWS = BN / CL;
-            if (B_MN == 0) {
-              tma_load_2d_mc(&tmB, full_bar + stage, sb + crank * ROWS * 128, kb * BK, n_blk * BN + crank * ROWS, kMask);
-            } else {
 #pragma unroll
-              for (int j = 0; j < ROWS / 64; ++j)
-                tma_load_2d_mc(&tmB, full_bar + stage, sb + (crank * (ROWS / 64) + j) * BOX_BYTES,
-                               n_blk * BN + crank * ROWS + j * 64, kb * BK, kMask);
-            }
+            for (int j = 0; j < BN / 64; ++j)
+              tma_load_2d(&tmB, full_bar + stage, sb + j * BOX_BYTES, n_blk * BN + j * 64, kb * BK);
           }
         }
         __syncwarp();
@@ -577,17 +556,12 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     }
   } else if (warp == MMA_WARP) {
     constexpr uint32_t idesc = make_idesc(BM, BN, A_MN, B_MN);
-    // descriptor = constant part | (smem address >> 4); K-major: +32 B per 16-element k-step inside the
-    // 128 B swizzle row, MN-major: +2 groups of 8 k-rows (2048 B)
-    const uint64_t da0 = A_MN == 0 ? smem_desc(0, 16, 1024) : smem_desc(0, BOX_BYTES, 1024);
-    const uint64_t db0 = B_MN == 0 ? smem_desc(0, 16, 1024) : smem_desc(0, BOX_BYTES, 1024);
-    constexpr uint32_t a_step = (A_MN == 0 ? 32 : 2048) >> 4, b_step = (B_MN == 0 ? 32 : 2048) >> 4;
     const uint32_t smem_base = smem_u32(smem);
     int stage = 0;
     uint32_t phase = 0;
     int acc = 0;
     uint32_t acc_phase = 0;
-    for (int tile = cluster_id; tile < total_tiles; tile += num_clusters) {
+    for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x) {
       const int split = (tile / p.m_groups) / p.n_tiles;
       const int kb0 = split * p.kb_per_split;
       const int kb1 = min(p.kb_total, kb0 + p.kb_per_split);
@@ -606,9 +580,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             const uint64_t db = B_MN == 0 ? smem_desc(sb + k * 32, 16, 1024) : smem_desc(sb + k * 2048, BOX_BYTES, 1024);
             umma_bf16(d_tmem, da, db, idesc, (kb > kb0 || k > 0) ? 1u : 0u);
           }
-          // frees the smem stage (in every CTA of the cluster) when the MMAs above have read it
-          if (CL == 1) umma_commit(empty_bar + stage);
-          else umma_commit_mc(empty_bar + stage, kMask);
+          umma_commit(empty_bar + stage);                    // frees the smem stage when the MMAs above have read it
           if (kb == kb1 - 1) umma_commit(tfull_bar + acc);  // accumulator complete
         }
         __syncwarp();
@@ -630,8 +602,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     uint32_t acc_phase = 0;
     const bool vec_ok = (p.epi.ldc % 4 == 0) && (!p.epi.aux || p.epi.ldaux % 4 == 0);
     float *stage = epi_stage + ew * EPI_STAGE_FLOATS;
-    for (int tile = cluster_id; tile < total_tiles; tile += num_clusters) {
-      const int m_blk = (tile % p.m_groups) * CL + crank;
+    for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x) {
+      const int m_blk = tile % p.m_groups;
       const int n_blk = (tile / p.m_groups) % p.n_tiles;
       const int row0 = m_blk * BM + quarter * 32;
       const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + acc * BN + half * 128;
@@ -656,23 +628,21 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   }
   tc_fence_before();
   __syncthreads();
-  if (CL > 1) cluster_sync_all();     // nobody leaves while a peer may still multicast into / arrive on this CTA
   if (warp == MMA_WARP) {
     tc_fence_after();
     tmem_dealloc(tmem_base, 512);
   }
 }
 
-
 // ---- CTA-pair kernel (tcgen05.mma.cta_group::2) ----------------------------------------------------
-// Same roles, epilogue and tile walk as gemm_tc_kernel<.., CL = 2>, but the two CTAs of a cluster form ONE
-// 256 x 256 MMA: each CTA stages its own 128 rows of A and HALF of the B tile (128 of the 256 n-rows); the leader
-// (cluster rank 0) issues every instruction for both tensor cores, which read the other half of B from the peer's
-// shared memory.  Per CTA and k-block that is 32 KB filled + 32 KB read instead of 48 + 48 (with the multicast
-// version every CTA still holds -- and its tensor core still reads -- the whole B tile): the 128 B/clk
-// shared-memory port is what this relieves (TMA fill 96 B/clk + operand reads 96 B/clk at full MMA rate in the
-// 1-CTA kernel).  Ring: 6 x 32 KB (the timeline showed the producer only ~2 k clk ahead of the MMAs with 5 stages,
-// about one L2 round trip: the first k-block of a tile arrived late).
+// The two CTAs of a cluster form ONE 256 x 256 MMA: each CTA stages its own 128 rows of A and HALF of the B tile (128 of
+// the 256 n-rows); the leader (cluster rank 0) issues every instruction for both tensor cores, which read the other half
+// of B from the peer's shared memory.  Per CTA and k-block that is 32 KB filled + 32 KB read instead of the 48 + 48 of a
+// 128 x 256 cta_group::1 tile (whose tensor core reads the whole B tile even when clusters share it by TMA multicast):
+// the 128 B/clk shared-memory port is what this relieves (TMA fill 96 B/clk + operand reads 96 B/clk at full MMA rate
+// with 1-CTA tiles).  With M <= 128 the peer's A rows are TMA zero fill.  Ring: 6 x 32 KB (the timeline showed the
+// producer only ~2 k clk ahead of the MMAs with 5 stages, about one L2 round trip: the first k-block of a tile arrived
+// late).
 // Protocol (as in DeepGEMM's sm_100 kernels): both producers report their TMA bytes to the LEADER's full barrier
 // (cp.async.bulk.tensor.cta_group::2 with a shared::cluster barrier address; arrival count 2 = leader's
 // arrive.expect_tx + the peer's plain arrive); tcgen05.commit.cta_group::2 multicasts "stage free" / "accumulator
@@ -680,8 +650,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
 constexpr int STAGES2 = 6;
 constexpr int B2_BYTES = (BN / 2) * BK * 2;           // 16 KB: this CTA's half of the B tile
 constexpr int STAGE2_BYTES = A_BYTES + B2_BYTES;      // 32 KB
-constexpr int EPI2_STAGE_BYTES = EPI_STAGE_BYTES;     // one 4 KB transposition buffer per epilogue warp
-constexpr int GEMM2_SMEM = STAGES2 * STAGE2_BYTES + EPI2_STAGE_BYTES + 1024 /*align*/ + 256 /*barriers*/;
+constexpr int GEMM2_SMEM = STAGES2 * STAGE2_BYTES + EPI_STAGE_BYTES + 1024 /*align*/ + 256 /*barriers*/;
 static_assert(GEMM2_SMEM <= 227 * 1024, "pair kernel: shared memory over the 227 KB limit");
 
 // EPI: -1 = every epilogue kind behind a run-time switch (any combination the C ABI allows); >= 0 = the kernel is compiled
@@ -696,7 +665,7 @@ gemm_tc_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
   extern __shared__ uint8_t smem_raw[];
   uint8_t *smem = reinterpret_cast<uint8_t *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
   float *epi_stage = reinterpret_cast<float *>(smem + STAGES2 * STAGE2_BYTES);
-  uint64_t *full_bar = reinterpret_cast<uint64_t *>(smem + STAGES2 * STAGE2_BYTES + EPI2_STAGE_BYTES);
+  uint64_t *full_bar = reinterpret_cast<uint64_t *>(smem + STAGES2 * STAGE2_BYTES + EPI_STAGE_BYTES);
   uint64_t *empty_bar = full_bar + STAGES2;
   uint64_t *tfull_bar = empty_bar + STAGES2;
   uint64_t *tempty_bar = tfull_bar + 2;
@@ -721,7 +690,7 @@ gemm_tc_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
     }
     fence_barrier_init();
   }
-  // Each CTA allocates ALL 512 columns of its own tensor memory (cta_group::1, as the 1-CTA kernel does): the base
+  // Each CTA allocates ALL 512 columns of its own tensor memory (cta_group::1): the base
   // address is then 0 in both CTAs of the pair, which is the symmetric layout cta_group::2 MMAs address.
   if (warp == MMA_WARP) tmem_alloc(tmem_slot, 512);
   tc_fence_before();
@@ -732,6 +701,11 @@ gemm_tc_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
 
   const int total_tiles = p.m_groups * p.n_tiles * p.splits;   // per pair: two adjacent m-tiles, one n-tile
 
+  // Producer and MMA roles run WARP-UNIFORMLY (all 32 lanes execute the loops and the barrier waits;
+  // only the TMA / tcgen05 instructions themselves sit under elect_one).  With the whole role under
+  // `if (lane == 0)` the loop state lives in per-thread registers and every TMA / MMA operand has
+  // to be moved to uniform registers through an ELECT / R2UR.BROADCAST waterfall loop: the MMA
+  // thread then needs ~100 issue cycles per 128-cycle MMA and the tensor pipe starves.
   if (warp == TMA_WARP) {
     int stage = 0;
     uint32_t phase = 0;
@@ -982,37 +956,24 @@ int sm_count() {
   return n;
 }
 
-template <int A_MN, int B_MN, int CL>
+template <int A_MN, int B_MN>
 static int launch_variant(const CUtensorMap &ta, const CUtensorMap &tb, const GemmTcParams &p, int grid, cudaStream_t st) {
   static bool configured = false;
   if (!configured) {
-    ASIS_CUDA(cudaFuncSetAttribute(gemm_tc_kernel<A_MN, B_MN, CL>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM));
+    ASIS_CUDA(cudaFuncSetAttribute(gemm_tc_kernel<A_MN, B_MN>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM));
     configured = true;
   }
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(grid);
-  cfg.blockDim = dim3(GEMM_THREADS);
-  cfg.dynamicSmemBytes = GEMM_SMEM;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = CL;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  ASIS_CUDA(cudaLaunchKernelEx(&cfg, gemm_tc_kernel<A_MN, B_MN, CL>, ta, tb, p));
+  gemm_tc_kernel<A_MN, B_MN><<<grid, GEMM_THREADS, GEMM_SMEM, st>>>(ta, tb, p);
   ASIS_LAUNCHED();
   return ASIS_OK;
 }
 
-template <int CL>
-static int launch_majors(int a_major, int b_major, const CUtensorMap &ta, const CUtensorMap &tb, const GemmTcParams &p,
+static int launch_single(int a_major, int b_major, const CUtensorMap &ta, const CUtensorMap &tb, const GemmTcParams &p,
                          int grid, cudaStream_t st) {
-  if (a_major == ASIS_MAJOR_K && b_major == ASIS_MAJOR_K) return launch_variant<0, 0, CL>(ta, tb, p, grid, st);
-  if (a_major == ASIS_MAJOR_K && b_major == ASIS_MAJOR_MN) return launch_variant<0, 1, CL>(ta, tb, p, grid, st);
-  if (a_major == ASIS_MAJOR_MN && b_major == ASIS_MAJOR_MN) return launch_variant<1, 1, CL>(ta, tb, p, grid, st);
-  return launch_variant<1, 0, CL>(ta, tb, p, grid, st);
+  if (a_major == ASIS_MAJOR_K && b_major == ASIS_MAJOR_K) return launch_variant<0, 0>(ta, tb, p, grid, st);
+  if (a_major == ASIS_MAJOR_K && b_major == ASIS_MAJOR_MN) return launch_variant<0, 1>(ta, tb, p, grid, st);
+  if (a_major == ASIS_MAJOR_MN && b_major == ASIS_MAJOR_MN) return launch_variant<1, 1>(ta, tb, p, grid, st);
+  return launch_variant<1, 0>(ta, tb, p, grid, st);
 }
 
 template <int A_MN, int B_MN, int EPI, int CDT, int AUX>
@@ -1064,26 +1025,6 @@ static int launch_pair(int a_major, int b_major, const CUtensorMap &ta, const CU
     return launch_pair_variant<1, 1, -1, -1, -1>(ta, tb, p, grid, st);
   }
   return launch_pair_variant<1, 0, -1, -1, -1>(ta, tb, p, grid, st);
-}
-
-// ASIS_GEMM_PAIR=0 falls back to the 1-CTA MMA kernel with B multicast (kept for comparison / bisecting)
-static bool pair_pref() {
-  static int v = -1;
-  if (v < 0) {
-    const char *e = getenv("ASIS_GEMM_PAIR");
-    v = e ? (atoi(e) != 0) : 1;
-  }
-  return v != 0;
-}
-
-static int cluster_pref() {
-  static int v = -1;
-  if (v < 0) {
-    const char *e = getenv("ASIS_GEMM_CLUSTER");
-    v = e ? atoi(e) : 2;
-    if (v != 1 && v != 2 && v != 4) v = 2;
-  }
-  return v;
 }
 
 // narrow outputs (the N = 64 / 128 convolutions and adapter projections): a 256-wide MMA would spend 4x / 2x the tensor
@@ -1182,8 +1123,7 @@ int gemm_tc_launch(const void *A, int a_major, int64_t lda, const void *B, int b
   p.n_tiles = (N + BN - 1) / BN;
   p.kb_total = (K + BK - 1) / BK;
   p.epi = epi;
-  int CL = cluster_pref();
-  while (CL > 1 && p.m_tiles < CL) CL >>= 1;     // nothing to share the B tile with
+  const int CL = p.m_tiles == 1 ? 1 : 2;        // CTAs per cluster: M <= 128 runs the 1-CTA kernel, the rest the pair kernel
   p.m_groups = (p.m_tiles + CL - 1) / CL;
   const int sms = sm_count();
   const int tiles = p.m_groups * CL * p.n_tiles;
@@ -1209,18 +1149,14 @@ int gemm_tc_launch(const void *A, int a_major, int64_t lda, const void *B, int b
   if (a_major == ASIS_MAJOR_K) rc = make_tmap_2d(&ta, A, K, M, lda, BK, BM);
   else rc = make_tmap_2d(&ta, A, M, K, lda, 64, BK);
   if (rc) return rc;
-  const bool pair = CL == 2 && pair_pref();
-  if (b_major == ASIS_MAJOR_K) rc = make_tmap_2d(&tb, B, K, N, ldb, BK, pair ? p.n_mma / 2 : BN / CL);   // one slice per CTA of the cluster
+  if (b_major == ASIS_MAJOR_K) rc = make_tmap_2d(&tb, B, K, N, ldb, BK, CL == 1 ? BN : p.n_mma / 2);   // a pair CTA loads half of the B tile
   else rc = make_tmap_2d(&tb, B, N, K, ldb, 64, BK);
   if (rc) return rc;
   const int cluster_tiles = p.m_groups * p.n_tiles * splits;
   int clusters = sms / CL;
   if (cluster_tiles < clusters) clusters = cluster_tiles;
-  const int grid = clusters * CL;
-  if (pair) return launch_pair(a_major, b_major, ta, tb, p, grid, st);
-  if (CL == 4) return launch_majors<4>(a_major, b_major, ta, tb, p, grid, st);
-  if (CL == 2) return launch_majors<2>(a_major, b_major, ta, tb, p, grid, st);
-  return launch_majors<1>(a_major, b_major, ta, tb, p, grid, st);
+  if (CL == 1) return launch_single(a_major, b_major, ta, tb, p, clusters, st);
+  return launch_pair(a_major, b_major, ta, tb, p, clusters * 2, st);
 }
 
 }  // namespace asis

@@ -5,8 +5,6 @@
 // LayerNorm: nn.LayerNorm(eps=1e-6) of the reference (dinov2/models/vision_transformer.py:89;
 // backbones/adapter_blocks.py:114).  Column sums: bias gradients of nn.Linear and the LayerScale
 // gamma gradient (dinov2/layers/layer_scale.py:26-27).
-#include <stdlib.h>
-
 #include "common.cuh"
 
 namespace asis {
@@ -68,100 +66,12 @@ __global__ void __launch_bounds__(kLnWarps * 32) ln_fwd_kernel(const XT *__restr
   }
 }
 
-// backward: warps stride over rows; per-lane partial dgamma/dbeta for the lane's columns, block
-// reduction through shared memory, one partial row per block -> workspace[block][2][C].
-// Each row is read twice (second read hits L1): pass 1 the two row sums, pass 2 dx and the column
-// partials -- keeping the row in registers instead costs ~200 registers/thread and one resident
-// block per SM, which measured 5x off the HBM roofline.
-template <typename DT, typename XT, int NV>
-__global__ void __launch_bounds__(kLnWarps * 32, 2) ln_bwd_kernel(const DT *__restrict__ dy, const XT *__restrict__ x,
-                                                                   const float *__restrict__ gamma,
-                                                                   const float *__restrict__ mean,
-                                                                   const float *__restrict__ rstd,
-                                                                   const float *__restrict__ dres, float *__restrict__ dx,
-                                                                   float *__restrict__ partial, int R, int C) {
-  __shared__ float red[kLnWarps][32 * 4 + 4];
-  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-  float dg[NV][4], db[NV][4];
-#pragma unroll
-  for (int j = 0; j < NV; ++j)
-#pragma unroll
-    for (int i = 0; i < 4; ++i) dg[j][i] = db[j][i] = 0.f;
-  for (int row = blockIdx.x * kLnWarps + wid; row < R; row += gridDim.x * kLnWarps) {
-    const float mu = mean[row], rs = rstd[row];
-    const DT *dyr = dy + (size_t)row * C;
-    const XT *xr = x + (size_t)row * C;
-    float s1 = 0.f, s2 = 0.f;
-#pragma unroll
-    for (int j = 0; j < NV; ++j) {
-      const int c = 4 * (lane + 32 * j);
-      if (c < C) {
-        float d[4], xv[4], g[4];
-        load4(dyr + c, d);
-        load4(xr + c, xv);
-        load4(gamma + c, g);
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-          const float t = d[i] * g[i];
-          s1 += t;
-          s2 += t * ((xv[i] - mu) * rs);
-        }
-      }
-    }
-    s1 = warp_sum(s1) / (float)C;
-    s2 = warp_sum(s2) / (float)C;
-    float *dxr = dx + (size_t)row * C;
-#pragma unroll
-    for (int j = 0; j < NV; ++j) {
-      const int c = 4 * (lane + 32 * j);
-      if (c < C) {
-        float d[4], xv[4], g[4], o[4];
-        load4(dyr + c, d);
-        load4(xr + c, xv);
-        load4(gamma + c, g);
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-          const float xh = (xv[i] - mu) * rs;
-          dg[j][i] += d[i] * xh;
-          db[j][i] += d[i];
-          o[i] = rs * (d[i] * g[i] - s1 - xh * s2);
-        }
-        if (dres) {
-          float r4[4];
-          load4(dres + (size_t)row * C + c, r4);
-#pragma unroll
-          for (int i = 0; i < 4; ++i) o[i] += r4[i];
-        }
-        store4(dxr + c, o);
-      }
-    }
-  }
-  // block reduction of the partials, one 128-column strip (index j) at a time
-  float *pg = partial + (size_t)blockIdx.x * 2 * C;
-  float *pb = pg + C;
-#pragma unroll
-  for (int j = 0; j < NV; ++j) {
-    for (int pass = 0; pass < 2; ++pass) {
-      __syncthreads();
-#pragma unroll
-      for (int i = 0; i < 4; ++i) red[wid][lane * 4 + i] = pass == 0 ? dg[j][i] : db[j][i];
-      __syncthreads();
-      if (threadIdx.x < 128) {
-        float t = 0.f;
-#pragma unroll
-        for (int w = 0; w < kLnWarps; ++w) t += red[w][threadIdx.x];
-        const int c = 128 * j + threadIdx.x;
-        if (c < C) (pass == 0 ? pg : pb)[c] = t;
-      }
-    }
-  }
-}
-
-// v2: a block owns kLn2Rows rows per iteration and a thread owns 4 columns (C <= 1024 = 256 x 4), so
-// the column partials d gamma / d beta are 8 registers instead of 64, every element is read once
+// backward: a block owns kLn2Rows rows per iteration and a thread owns 4 columns (C <= 1024 = 256 x 4), so
+// the column partials d gamma / d beta are 8 registers per thread, every element is read once
 // (row data stays in registers between the row reduction and the dx pass), and the loads of all
 // kLn2Rows rows are in flight together.  Row sums: warp shuffles, then one shared-memory exchange per
-// iteration (double buffered: one __syncthreads per kLn2Rows rows).
+// iteration (double buffered: one __syncthreads per kLn2Rows rows).  Each block writes one partial
+// row -> workspace[block][2][C].
 // Tuning knobs (A/B builds, tools/ln_variants.sh, profiles/r2y_ln_variants.md): rows per block iteration and resident
 // blocks per SM (= grid / 148).  4 rows x 3 blocks (80 registers, 28-40 bytes of spills) was the first setting: 78.9 us
 // for [21168 x 1024] with the fused residual gradient; 2 rows x 4 blocks (59 registers, no spills): 68.6 us = 4.4 TB/s,
@@ -542,20 +452,14 @@ extern "C" int asis_layernorm_backward(const void *dy, int dy_dtype, const void 
   ASIS_REQUIRE(dy && x && gamma && mean && rstd && dx && workspace, "layernorm_backward: null pointer");
   ASIS_REQUIRE(dtype_ok(dy_dtype) && dtype_ok(x_dtype), "layernorm_backward: bad dtype");
   ASIS_REQUIRE(R > 0 && C > 0 && C % 4 == 0, "layernorm_backward: C=%d must be a positive multiple of 4", C);
-  const int nv = ln_nv(C);
-  if (!nv) ASIS_FAIL(ASIS_ERR_UNSUPPORTED, "layernorm_backward: C=%d > 1024 not supported", C);
+  if (C > 1024) ASIS_FAIL(ASIS_ERR_UNSUPPORTED, "layernorm_backward: C=%d > 1024 not supported", C);   // 256 threads x 4 columns
   const size_t need = asis_layernorm_backward_workspace_bytes(R, C);
   if (workspace_bytes < need) ASIS_FAIL(ASIS_ERR_WORKSPACE, "layernorm_backward: workspace %zu < %zu bytes", workspace_bytes, need);
   ASIS_REQUIRE(aligned16(dy) && aligned16(x) && aligned16(dx) && aligned16(gamma) && aligned16(workspace) && (!dres || aligned16(dres)), "layernorm_backward: pointers must be 16-byte aligned");
   cudaStream_t st = (cudaStream_t)stream;
   const int blocks = ln_bwd_blocks(R);
   float *partial = (float *)workspace;
-  static const bool use_v1 = getenv("ASIS_LN_BWD_V1") != nullptr;   // A/B switch for tools/one_kernel.py
-  if (use_v1) {
-    ASIS_DISPATCH_DTYPE(dy_dtype, DT, ASIS_DISPATCH_DTYPE(x_dtype, XT, LN_NV_SWITCH(nv, (ln_bwd_kernel<DT, XT, NV><<<blocks, kLnWarps * 32, 0, st>>>((const DT *)dy, (const XT *)x, gamma, mean, rstd, dres, dx, partial, R, C)))));
-  } else {
-    ASIS_DISPATCH_DTYPE(dy_dtype, DT, ASIS_DISPATCH_DTYPE(x_dtype, XT, (ln_bwd2_kernel<DT, XT><<<blocks, 256, 0, st>>>((const DT *)dy, (const XT *)x, gamma, mean, rstd, dres, dx, partial, R, C))));
-  }
+  ASIS_DISPATCH_DTYPE(dy_dtype, DT, ASIS_DISPATCH_DTYPE(x_dtype, XT, (ln_bwd2_kernel<DT, XT><<<blocks, 256, 0, st>>>((const DT *)dy, (const XT *)x, gamma, mean, rstd, dres, dx, partial, R, C))));
   ASIS_LAUNCHED();
   if (dgamma && dbeta) {
     launch_reduce_partials(partial, blocks, 2 * C, dgamma, dbeta, C, accumulate, st);

@@ -105,16 +105,7 @@ __device__ __forceinline__ void bulk_load_1d(uint64_t *bar, void *dst, const voi
                : "memory");
 }
 
-// multicast: the box lands at the same CTA-relative smem offset in every CTA of `mask`, and each
-// destination CTA's mbarrier (same offset) receives the complete_tx
-__device__ __forceinline__ void tma_load_2d_mc(const CUtensorMap *m, uint64_t *bar, void *dst, int c0, int c1, uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4}], [%2], %5;"
-      ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "h"(mask)
-      : "memory");
-}
-
-// 2-CTA pair variants (cta_group::2): the destination is this CTA's shared memory, the mbarrier may live in the
+// 2-D load of a 2-CTA pair (cta_group::2): the destination is this CTA's shared memory, the mbarrier may live in the
 // PEER CTA (shared::cluster address from mapa) -- both CTAs of a pair report their bytes to the leader's barrier
 __device__ __forceinline__ void tma_load_2d_pair(const CUtensorMap *m, uint32_t bar_cluster_addr, void *dst, int c0, int c1) {
   asm volatile(
@@ -230,11 +221,6 @@ __device__ __forceinline__ void umma_commit_pair(uint64_t *bar, uint16_t mask) {
 // all previously issued MMAs of this thread arrive on the mbarrier when they complete
 __device__ __forceinline__ void umma_commit(uint64_t *bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-
-// same, arriving on the mbarrier at this smem offset in every CTA of `mask`
-__device__ __forceinline__ void umma_commit_mc(uint64_t *bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(smem_u32(bar)), "h"(mask) : "memory");
 }
 
 // 32 lanes x 32 columns of fp32: thread i of the warp gets lane (base_lane + i), columns [c, c+32).

@@ -45,55 +45,57 @@ def test_gemm_tc_majors(M, N, K_, am, bm):
 
 
 def test_gemm_tc_split_k_weight_gradient():
-    torch.manual_seed(1)
-    R, N, K_ = 21180, 1024, 1024                 # ViT-L proj weight gradient: 32 tiles, K = tokens
-    dy = torch.randn(R, N, device=DEV).bfloat16()
-    x = torch.randn(R, K_, device=DEV).bfloat16()
-    ref = dy.float().t() @ x.float()
-    dw, _ = K.gemm(BF16, dy, MAJOR_MN, x, MAJOR_MN, N, K_, R, torch.float32)
-    assert relerr(dw, ref) < GEMM_TOL
-    acc = torch.ones(N, K_, device=DEV)
-    dw2, _ = K.gemm(BF16, dy, MAJOR_MN, x, MAJOR_MN, N, K_, R, torch.float32, epilogue=EPI_ACCUMULATE, out=acc)
-    assert relerr(dw2, ref + 1) < GEMM_TOL
+    for R, N, K_ in ((21180, 1024, 1024),       # ViT-L proj weight gradient: 32 tiles, K = tokens
+                     (21168, 96, 1024)):        # a weight gradient of the step with one M tile (1-CTA kernel)
+        torch.manual_seed(1)
+        dy = torch.randn(R, N, device=DEV).bfloat16()
+        x = torch.randn(R, K_, device=DEV).bfloat16()
+        ref = dy.float().t() @ x.float()
+        dw, _ = K.gemm(BF16, dy, MAJOR_MN, x, MAJOR_MN, N, K_, R, torch.float32)
+        assert relerr(dw, ref) < GEMM_TOL
+        acc = torch.ones(N, K_, device=DEV)
+        dw2, _ = K.gemm(BF16, dy, MAJOR_MN, x, MAJOR_MN, N, K_, R, torch.float32, epilogue=EPI_ACCUMULATE, out=acc)
+        assert relerr(dw2, ref + 1) < GEMM_TOL
 
 
 def test_gemm_tc_epilogues():
-    torch.manual_seed(2)
-    M, N, K_ = 1000, 1024, 512
-    A = torch.randn(M, K_, device=DEV).bfloat16()
-    B = torch.randn(N, K_, device=DEV).bfloat16()
-    ref = A.float() @ B.float().t()
-    bias = torch.randn(N, device=DEV)
-    gamma = torch.randn(N, device=DEV)
-    res = torch.randn(M, N, device=DEV)
-    c, _ = K.gemm(BF16, A, MAJOR_K, B, MAJOR_K, M, N, K_, torch.bfloat16, bias=bias)
-    assert relerr(c.float(), ref + bias) < TOL
-    c, aux = K.gemm(BF16, A, MAJOR_K, B, MAJOR_K, M, N, K_, torch.bfloat16, epilogue=EPI_GELU, bias=bias,
-                    want_aux_dtype=torch.bfloat16)
-    assert relerr(c.float(), torch.nn.functional.gelu(ref + bias)) < TOL and relerr(aux.float(), ref + bias) < TOL
-    c, aux = K.gemm(BF16, A, MAJOR_K, B, MAJOR_K, M, N, K_, torch.float32, epilogue=EPI_SCALE_RESIDUAL, bias=bias,
-                    gamma=gamma, residual=res, want_aux_dtype=torch.bfloat16)
-    assert relerr(c, res + gamma * (ref + bias)) < GEMM_TOL and relerr(aux.float(), ref + bias) < TOL
-    h = torch.randn(M, N, device=DEV).bfloat16()
-    hh = h.float().requires_grad_(True)
-    (dg,) = torch.autograd.grad(torch.nn.functional.gelu(hh), hh, torch.ones_like(hh))
-    c, _ = K.gemm(BF16, A, MAJOR_K, B, MAJOR_K, M, N, K_, torch.float32, epilogue=EPI_DGELU, aux=h)
-    assert relerr(c, ref * dg) < GEMM_TOL
-    # GELU with the derivative saved for the backward, and the backward epilogue that multiplies by it
-    pre = (ref + bias).requires_grad_(True)
-    (dpre,) = torch.autograd.grad(torch.nn.functional.gelu(pre), pre, torch.ones_like(pre))
-    c, aux = K.gemm(BF16, A, MAJOR_K, B, MAJOR_K, M, N, K_, torch.bfloat16, epilogue=EPI_GELU_GRAD, bias=bias,
-                    want_aux_dtype=torch.bfloat16)
-    assert relerr(c.float(), torch.nn.functional.gelu(ref + bias)) < TOL and relerr(aux.float(), dpre) < TOL
-    c, _ = K.gemm(BF16, A, MAJOR_K, B, MAJOR_K, M, N, K_, torch.bfloat16, epilogue=EPI_MUL_AUX, aux=aux)
-    assert relerr(c.float(), ref * aux.float()) < TOL
-    # the same two on a shape with M / N tails (generic epilogue path)
-    Mt, Nt = 333, 200
-    c, aux = K.gemm(BF16, A[:Mt], MAJOR_K, B[:Nt], MAJOR_K, Mt, Nt, K_, torch.bfloat16, epilogue=EPI_GELU_GRAD, bias=bias[:Nt],
-                    want_aux_dtype=torch.bfloat16)
-    assert relerr(c.float(), torch.nn.functional.gelu(ref[:Mt, :Nt] + bias[:Nt])) < TOL and relerr(aux.float(), dpre[:Mt, :Nt]) < TOL
-    c, _ = K.gemm(BF16, A[:Mt], MAJOR_K, B[:Nt], MAJOR_K, Mt, Nt, K_, torch.float32, epilogue=EPI_MUL_AUX, aux=aux)
-    assert relerr(c, ref[:Mt, :Nt] * aux.float()) < GEMM_TOL
+    for M, Mt in ((1000, 333), (96, 77)):      # M <= 128: one M tile (1-CTA kernel)
+        torch.manual_seed(2)
+        N, K_ = 1024, 512
+        A = torch.randn(M, K_, device=DEV).bfloat16()
+        B = torch.randn(N, K_, device=DEV).bfloat16()
+        ref = A.float() @ B.float().t()
+        bias = torch.randn(N, device=DEV)
+        gamma = torch.randn(N, device=DEV)
+        res = torch.randn(M, N, device=DEV)
+        c, _ = K.gemm(BF16, A, MAJOR_K, B, MAJOR_K, M, N, K_, torch.bfloat16, bias=bias)
+        assert relerr(c.float(), ref + bias) < TOL
+        c, aux = K.gemm(BF16, A, MAJOR_K, B, MAJOR_K, M, N, K_, torch.bfloat16, epilogue=EPI_GELU, bias=bias,
+                        want_aux_dtype=torch.bfloat16)
+        assert relerr(c.float(), torch.nn.functional.gelu(ref + bias)) < TOL and relerr(aux.float(), ref + bias) < TOL
+        c, aux = K.gemm(BF16, A, MAJOR_K, B, MAJOR_K, M, N, K_, torch.float32, epilogue=EPI_SCALE_RESIDUAL, bias=bias,
+                        gamma=gamma, residual=res, want_aux_dtype=torch.bfloat16)
+        assert relerr(c, res + gamma * (ref + bias)) < GEMM_TOL and relerr(aux.float(), ref + bias) < TOL
+        h = torch.randn(M, N, device=DEV).bfloat16()
+        hh = h.float().requires_grad_(True)
+        (dg,) = torch.autograd.grad(torch.nn.functional.gelu(hh), hh, torch.ones_like(hh))
+        c, _ = K.gemm(BF16, A, MAJOR_K, B, MAJOR_K, M, N, K_, torch.float32, epilogue=EPI_DGELU, aux=h)
+        assert relerr(c, ref * dg) < GEMM_TOL
+        # GELU with the derivative saved for the backward, and the backward epilogue that multiplies by it
+        pre = (ref + bias).requires_grad_(True)
+        (dpre,) = torch.autograd.grad(torch.nn.functional.gelu(pre), pre, torch.ones_like(pre))
+        c, aux = K.gemm(BF16, A, MAJOR_K, B, MAJOR_K, M, N, K_, torch.bfloat16, epilogue=EPI_GELU_GRAD, bias=bias,
+                        want_aux_dtype=torch.bfloat16)
+        assert relerr(c.float(), torch.nn.functional.gelu(ref + bias)) < TOL and relerr(aux.float(), dpre) < TOL
+        c, _ = K.gemm(BF16, A, MAJOR_K, B, MAJOR_K, M, N, K_, torch.bfloat16, epilogue=EPI_MUL_AUX, aux=aux)
+        assert relerr(c.float(), ref * aux.float()) < TOL
+        # the same two on a shape with M / N tails (generic epilogue path)
+        Nt = 200
+        c, aux = K.gemm(BF16, A[:Mt], MAJOR_K, B[:Nt], MAJOR_K, Mt, Nt, K_, torch.bfloat16, epilogue=EPI_GELU_GRAD, bias=bias[:Nt],
+                        want_aux_dtype=torch.bfloat16)
+        assert relerr(c.float(), torch.nn.functional.gelu(ref[:Mt, :Nt] + bias[:Nt])) < TOL and relerr(aux.float(), dpre[:Mt, :Nt]) < TOL
+        c, _ = K.gemm(BF16, A[:Mt], MAJOR_K, B[:Nt], MAJOR_K, Mt, Nt, K_, torch.float32, epilogue=EPI_MUL_AUX, aux=aux)
+        assert relerr(c, ref[:Mt, :Nt] * aux.float()) < GEMM_TOL
 
 
 @pytest.mark.parametrize("B,T,H", [(1, 128, 1), (2, 300, 3), (1, 1765, 16), (3, 1764, 2)])

@@ -1,5 +1,5 @@
 """Attention kernel microbench at the step's shape (B=12, T=1765, H=16, hd=64): forward and backward, CUDA events,
-median of N, checked against fp32 math on one (image, head) slice.  ASIS_ATTN_FWD=7 selects the previous forward."""
+median of N, checked against fp32 math on one (image, head) slice."""
 import json
 import os
 import sys
@@ -47,5 +47,4 @@ out2, lse2 = K.attention_forward(BF16, qkv, B, T, H, 64)
 fl = 4.0 * B * H * T * T * 64
 print(json.dumps(dict(B=B, T=T, H=H, fwd_us=round(tf * 1e3, 1), fwd_tflops=round(fl / tf / 1e9, 1), bwd_us=round(tb * 1e3, 1),
                       bwd_tflops_alg=round(2.5 * fl / tb / 1e9, 1), out_relerr=round(err, 5), lse_abserr=round(lerr, 6),
-                      finite=bool(torch.isfinite(out.float()).all()), repeatable=bool(torch.equal(out, out2) and torch.equal(lse, lse2)),
-                      fwd_version=os.environ.get("ASIS_ATTN_FWD", "8"))))
+                      finite=bool(torch.isfinite(out.float()).all()), repeatable=bool(torch.equal(out, out2) and torch.equal(lse, lse2)))))

@@ -1,10 +1,5 @@
 """Per-shape microbench of the tcgen05 GEMM on the shapes of the ViT-L/14 training step (the rows of
-`bench.py --detail`): TFLOP/s per launch, CUDA events on the launching stream, inputs larger than L2.
-Run once per kernel variant (the variant is chosen by environment variables read at first launch):
-
-    ASIS_GEMM_PAIR=0 python tools/gemm_bench.py      # 1-CTA MMA, B multicast
-    ASIS_GEMM_PAIR=1 python tools/gemm_bench.py      # CTA-pair MMA (default)
-"""
+`bench.py --detail`): TFLOP/s per launch, CUDA events on the launching stream, inputs larger than L2."""
 import json
 import os
 import sys
@@ -86,7 +81,7 @@ def main():
         rows.append(row)
         print(json.dumps(row), flush=True)
     tot = sum(r["us"] for r in rows)
-    print(json.dumps(dict(variant=dict(pair=os.environ.get("ASIS_GEMM_PAIR", "1")), total_us=round(tot, 1))), flush=True)
+    print(json.dumps(dict(total_us=round(tot, 1))), flush=True)
 
 
 if __name__ == "__main__":

@@ -107,7 +107,6 @@ def timeit(fn, iters=10):
 
 def perf():
     R = 21180
-    print("cluster =", os.environ.get("ASIS_GEMM_CLUSTER", "default(2)"))
     for tag, M, N, Kd, am, bm, odt in [
             ("qkv fwd K/K", R, 3072, 1024, MAJOR_K, MAJOR_K, torch.bfloat16),
             ("proj fwd K/K", R, 1024, 1024, MAJOR_K, MAJOR_K, torch.bfloat16),
