@@ -169,8 +169,12 @@ def gemm(compute, A, a_major, B, b_major, M, N, K, out_dtype, epilogue=EPI_NONE,
     if epilogue in (EPI_GELU, EPI_SCALE_RESIDUAL, EPI_GELU_GRAD) and aux is None and want_aux_dtype is not None:
         aux = torch.empty(M, N, dtype=want_aux_dtype, device=dev)
     if residual is not None:
-        residual = _c(residual)
         assert residual.dtype == torch.float32 and residual.shape[-1] == N
+        # the kernels read the residual with C's row pitch (ldc): a residual laid out like `out` is passed as it is
+        if residual.dim() != 2 or residual.stride() != (out.stride(0), 1):
+            if out.stride(0) != N:
+                raise ValueError(f"gemm: the residual must have out's row pitch {out.stride(0)} (strides {residual.stride()})")
+            residual = residual.contiguous()
     detail = None
     if _PROF[0] is not None:
         detail = (f"M={M} N={N} K={K} {'KM'[a_major]}/{'KM'[b_major]} epi={epilogue} out={'bf16' if out.dtype == torch.bfloat16 else 'f32'}"
