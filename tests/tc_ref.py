@@ -29,7 +29,10 @@ The exact quantities (which terms, which shadows) are written next to each refer
 `check` returns the largest err / bound ratio, where it is and the largest ratio of every slab (an output tile of
 the GEMM, an (image, head) of the attention), so a failure names the unit that went wrong.
 """
+import json
 import math
+import os
+import tempfile
 
 import torch
 
@@ -86,7 +89,8 @@ def slab_max(r, block):
 
 def check(name, out, ref, u, terms, block=None):
     """Elementwise |out - ref| <= u |ref| + sum c * shadow over `terms` = [(c, shadow), ...] (c and shadow broadcast
-    against ref).  Non-finite kernel values count as an infinite ratio."""
+    against ref).  Non-finite kernel values count as an infinite ratio.  `block`: the slab shape for slab_max, or a
+    function from the ratio tensor to the per-slab maxima."""
     out64 = out.detach().to(device=ref.device, dtype=torch.float64)
     err = (out64 - ref).abs()
     bound = u * ref.abs()
@@ -97,9 +101,37 @@ def check(name, out, ref, u, terms, block=None):
     ratio = torch.where(torch.isfinite(out64), ratio, torch.full_like(ratio, math.inf))
     i = int(ratio.flatten().argmax())
     where = tuple(int(x) for x in torch.unravel_index(torch.tensor(i), ratio.shape))
-    slabs = slab_max(ratio, block).cpu() if block is not None else None
+    slabs = None if block is None else (block(ratio) if callable(block) else slab_max(ratio, block)).cpu()
     return Report(name, float(ratio.flatten()[i]), where, float(err.flatten()[i]), float(bound.flatten()[i]),
                   float(ref.flatten()[i]), float(out64.flatten()[i]), slabs)
+
+
+# ---------------------------------------------------------------------------------------------- the trace
+def traced(fn):
+    """Run fn under torch.profiler; return (its result, [(kernel name, grid)] of the project's kernels)."""
+    from torch.profiler import ProfilerActivity, profile
+    with profile(activities=[ProfilerActivity.CPU, ProfilerActivity.CUDA]) as prof:
+        r = fn()
+        torch.cuda.synchronize()
+    with tempfile.TemporaryDirectory() as d:
+        path = os.path.join(d, "trace.json")
+        prof.export_chrome_trace(path)
+        with open(path) as f:
+            ev = json.load(f)["traceEvents"]
+    ks = [(e["name"].replace(" ", "").replace("(int)", ""), tuple(e.get("args", {}).get("grid", ()))) for e in ev
+          if e.get("cat") == "kernel" and "asis::" in e.get("name", "")]
+    return r, ks
+
+
+def expect_kernel(ks, pattern, grid):
+    """The one launch whose name contains `pattern` (spaces ignored) and its grid == `grid` (a tuple)."""
+    pat = pattern.replace(" ", "")
+    hits = [k for k in ks if pat in k[0]]
+    assert len(hits) == 1, f"expected one launch of {pattern}, trace has {[k[0] for k in ks]}"
+    name, g = hits[0]
+    assert g, f"the trace records no grid for {name}"
+    assert tuple(g) + (1,) * (3 - len(g)) == tuple(grid) + (1,) * (3 - len(grid)), (name, g, grid)
+    return name
 
 
 # ------------------------------------------------------------------------------------------------- GEMM

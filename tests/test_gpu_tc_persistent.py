@@ -5,10 +5,7 @@ barrier phases, TMEM double buffers and prefetches that only run from a CTA's se
 carry a scale or offset per M tile / (image, head), so a unit that reads another unit's data fails in its own slab.
 Each case prints the kernel, its units per CTA (cluster for the pair kernel), the rescale counts and the largest
 err / bound ratio."""
-import json
 import math
-import os
-import tempfile
 import time
 
 import pytest
@@ -26,33 +23,6 @@ BF, F32 = torch.bfloat16, torch.float32
 
 def sms():
     return torch.cuda.get_device_properties(0).multi_processor_count
-
-
-def traced(fn):
-    """Run fn under torch.profiler; return (its result, [(kernel name, grid)] of the project's kernels)."""
-    from torch.profiler import ProfilerActivity, profile
-    with profile(activities=[ProfilerActivity.CPU, ProfilerActivity.CUDA]) as prof:
-        r = fn()
-        torch.cuda.synchronize()
-    with tempfile.TemporaryDirectory() as d:
-        path = os.path.join(d, "trace.json")
-        prof.export_chrome_trace(path)
-        with open(path) as f:
-            ev = json.load(f)["traceEvents"]
-    ks = [(e["name"].replace(" ", "").replace("(int)", ""), tuple(e.get("args", {}).get("grid", ()))) for e in ev
-          if e.get("cat") == "kernel" and "asis::" in e.get("name", "")]
-    return r, ks
-
-
-def expect_kernel(ks, pattern, grid):
-    """The one launch whose name contains `pattern` (spaces ignored) and its grid == `grid` (a tuple)."""
-    pat = pattern.replace(" ", "")
-    hits = [k for k in ks if pat in k[0]]
-    assert len(hits) == 1, f"expected one launch of {pattern}, trace has {[k[0] for k in ks]}"
-    name, g = hits[0]
-    assert g, f"the trace records no grid for {name}"
-    assert tuple(g) + (1,) * (3 - len(g)) == tuple(grid) + (1,) * (3 - len(grid)), (name, g, grid)
-    return name
 
 
 # ------------------------------------------------------------------------------------------------- GEMM
@@ -142,9 +112,9 @@ def run_gemm_case(name, M, N, K_, am, bm, epi, odt, has_bias, aux_mode, kern, ld
     a, b = _lay(A, am), _lay(B, bm)
     launch = gemm_launch(M, N, K_, odt == F32, epi, has_bias)
     t0 = time.time()
-    (c, aux), ks = traced(lambda: K.gemm(BF16, a, am, b, bm, M, N, K_, odt, epilogue=epi, bias=bias, gamma=gamma, out=out,
+    (c, aux), ks = R.traced(lambda: K.gemm(BF16, a, am, b, bm, M, N, K_, odt, epilogue=epi, bias=bias, gamma=gamma, out=out,
                                          **kw))
-    kname = expect_kernel(ks, kern, (launch["grid"],))
+    kname = R.expect_kernel(ks, kern, (launch["grid"],))
     refs = R.gemm_ref(A, B, EPI_NAME[epi], bias=bias, gamma=gamma, residual=res, aux=aux_in, c_old=c_old,
                       splits=launch["splits"])
     reps = [R.check("c", c, refs["c"][0], R.u_out(odt), refs["c"][1], block=(128, 256))]
@@ -223,12 +193,12 @@ def test_attention_persistent(Bn, T, H, kind):
     qkv = R.attention_inputs(kind, Bn, T, H, g).to(DEV).bfloat16()
     dout = torch.randn(Bn, T, H * 64, generator=g).to(DEV).bfloat16()
     items, grid, npair = R.attn_units(Bn, T, H, sms())
-    (out, lse), ks = traced(lambda: K.attention_forward(BF16, qkv, Bn, T, H, 64))
-    kf = expect_kernel(ks, "attn_fwd8_kernel", (grid,))
-    dqkv, ks = traced(lambda: K.attention_backward(BF16, qkv, out, lse, dout, Bn, T, H, 64))
+    (out, lse), ks = R.traced(lambda: K.attention_forward(BF16, qkv, Bn, T, H, 64))
+    kf = R.expect_kernel(ks, "attn_fwd8_kernel", (grid,))
+    dqkv, ks = R.traced(lambda: K.attention_backward(BF16, qkv, out, lse, dout, Bn, T, H, 64))
     nqb = -(-T // 128)
-    expect_kernel(ks, "attn_bwd_dkdv_kernel", (nqb, H, Bn))
-    expect_kernel(ks, "attn_bwd_dq_kernel", (nqb, H, Bn))
+    R.expect_kernel(ks, "attn_bwd_dkdv_kernel", (nqb, H, Bn))
+    R.expect_kernel(ks, "attn_bwd_dq_kernel", (nqb, H, Bn))
     if items >= 2 * sms():
         assert grid < items
 
@@ -327,8 +297,8 @@ def test_conv3x3_persistent(Bn, H, W, Cin, Cout):
     msg = []
     for name, op, run, view, kern, u in outs:
         launch = conv_launch(op, Bn, H, W, Cin, Cout)
-        _, ks = traced(run)
-        expect_kernel(ks, kern, (launch["grid"],))
+        _, ks = R.traced(run)
+        R.expect_kernel(ks, kern, (launch["grid"],))
         ref, sh = refs[name]
         c = R.c_mma(launch["k"], launch["splits"]) + (R.C_EPI if op == 0 else 0.0)
         rep = R.check(name, view(), ref, u, [(c, sh)])
