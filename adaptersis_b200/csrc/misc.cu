@@ -450,6 +450,9 @@ extern "C" int asis_dwconv3x3_backward(const void *dy, const void *pre, const vo
   ASIS_REQUIRE(!fuse_gelu || pre, "dwconv_backward: fused GELU needs the saved pre-activation");
   ASIS_REQUIRE(dtype_ok(dtype), "dwconv_backward: bad dtype");
   ASIS_REQUIRE(B > 0 && C > 0 && C % 4 == 0, "dwconv_backward: C=%d must be a positive multiple of 4", C);
+  // 4-channel vector loads and stores of dy, pre, x, dx and of the GELU' buffer inside the workspace
+  ASIS_REQUIRE(aligned16(dy) && aligned16(x) && aligned16(dx) && aligned16(workspace) && (!pre || aligned16(pre)),
+               "dwconv_backward: pointers must be 16-byte aligned");
   Maps mp;
   if (int rc = make_maps(mp, n_maps, hs_host, ws_host)) return rc;
   const int ntok = mp.start[kMaxMaps];

@@ -187,7 +187,8 @@ int asis_patchify(const float *img, void *cols, int out_dtype, int B, int Cin, i
  *   x [B, n_tok, C] holding `n_maps` maps back to back (map i is hs[i] x ws[i]); stride 1, pad 1,
  *   weight [C, 3, 3] f32, bias [C] f32; optional fused exact GELU on the output.
  *   hs_host/ws_host are HOST arrays.  C % 4 == 0 and C <= 1280 (the forward stages the nine taps of all
- *   channels in 36 C bytes of shared memory); 1..4 maps. */
+ *   channels in 36 C bytes of shared memory); 1..4 maps.  x, y, pre, bias (forward) and dy, pre, x, dx,
+ *   workspace (backward) must be 16-byte aligned. */
 int asis_dwconv3x3_forward(const void *x, int dtype, const float *weight, const float *bias,
                            void *pre, void *y, int B, int C, int n_maps, const int *hs_host,
                            const int *ws_host, int fuse_gelu, void *stream);

@@ -134,6 +134,29 @@ def expect_kernel(ks, pattern, grid):
     return name
 
 
+# -------------------------------------------------------------------------------------- the output guards
+NAN_BITS = {2: 0x7fcb, 4: 0x7fc00bad}
+GUARD = 64
+
+
+def bits(t):
+    return t.view(torch.int16 if t.element_size() == 2 else torch.int32)
+
+
+def guarded(shape, dtype, device="cuda"):
+    """(buffer, view): `view` of `shape` inside a NaN-filled buffer with GUARD elements on each side."""
+    n = math.prod(shape)
+    buf = torch.empty(n + 2 * GUARD, dtype=dtype, device=device)
+    bits(buf).fill_(NAN_BITS[buf.element_size()])
+    return buf, buf[GUARD:GUARD + n].view(shape)
+
+
+def guards_intact(buf):
+    b = bits(buf)
+    nan = NAN_BITS[buf.element_size()]
+    return bool((b[:GUARD] == nan).all()) and bool((b[-GUARD:] == nan).all())
+
+
 # ------------------------------------------------------------------------------------------------- GEMM
 def _gelu(h):
     return 0.5 * h * (1.0 + torch.erf(h * 0.5 ** 0.5))

@@ -154,6 +154,25 @@ def test_host_side_validation_last_build_entry_points():
     assert rc != 0 and b"1024" in lib.asis_last_error()
 
 
+def test_dwconv_backward_refuses_misaligned_pointers():
+    """The depth-wise convolution backward loads and stores 4-channel vectors of dy, pre, x and dx (and of the GELU'
+    buffer in the workspace): a pointer off the 16-byte grid is refused on the host, before any launch."""
+    import ctypes
+    from adaptersis_b200 import _lib
+    lib = _lib.load()
+    fake, odd = ctypes.c_void_p(256), ctypes.c_void_p(260)
+    hs = (ctypes.c_int * 2)(7, 4)
+    ws = (ctypes.c_int * 2)(5, 3)
+    need = lib.asis_dwconv3x3_backward_workspace_bytes(2, 64, 47)
+    for dtype in (0, 1):
+        for i in range(5):                       # dy, pre, x, dx, workspace
+            p = [fake] * 5
+            p[i] = odd
+            rc = lib.asis_dwconv3x3_backward(p[0], p[1], p[2], dtype, fake, p[3], fake, fake, 0, 2, 64, 2, hs, ws, 1,
+                                             p[4], need, None)
+            assert rc == -1 and b"16-byte aligned" in lib.asis_last_error(), i
+
+
 def test_no_cpu_fallback():
     import adaptersis_b200 as asis
     m = asis.MSDeformAttn(d_model=32, n_levels=1, n_heads=4, n_points=2)

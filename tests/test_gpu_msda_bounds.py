@@ -4,7 +4,6 @@ edges and far outside.  Every case asserts from the torch.profiler trace which i
 launcher's arithmetic below), prints the launches and the worst err / bound ratio with where it occurred, and the
 backward is run twice and must be bit-identical.  The sweep calls the C ABI with each output inside a NaN-filled
 buffer: nothing outside the outputs may change."""
-import math
 import time
 
 import pytest
@@ -14,6 +13,7 @@ import msda_ref as MR
 import tc_ref as R
 from adaptersis_b200 import _lib, kernels as K
 from adaptersis_b200._lib import ptr
+from tc_ref import bits, guarded, guards_intact
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda"
@@ -79,28 +79,6 @@ def report(tag, reps, plan, t0):
           f"max err/bound {worst.ratio:.3g} ({worst.name} at {worst.where}) [{time.time() - t0:.1f} s]")
     for r in reps:
         assert r.ok, f"[{tag}] {r}"
-
-
-def bits(t):
-    return t.view(torch.int16 if t.element_size() == 2 else torch.int32)
-
-
-NAN_BITS = {2: 0x7fcb, 4: 0x7fc00bad}
-GUARD = 64
-
-
-def guarded(shape, dtype):
-    """(buffer, view): `view` of `shape` inside a NaN-filled buffer with GUARD elements on each side."""
-    n = math.prod(shape)
-    buf = torch.empty(n + 2 * GUARD, dtype=dtype, device=DEV)
-    bits(buf).fill_(NAN_BITS[buf.element_size()])
-    return buf, buf[GUARD:GUARD + n].view(shape)
-
-
-def guards_intact(buf):
-    b = bits(buf)
-    nan = NAN_BITS[buf.element_size()]
-    return bool((b[:GUARD] == nan).all()) and bool((b[-GUARD:] == nan).all())
 
 
 def abi_forward(value, ss, lsi, loc, aw):
